@@ -16,7 +16,7 @@ A "step" = one pass of the keyframe hot path over a batch of `--frames` syntheti
   --impl reference : the reference's own CPU code (oracle/_ref, SIMD build, one process per
           usable host core) on whole 4K frames of the same workload
 
-Prints ONE JSON line (rank 0).
+Prints ONE JSON line (rank 0).  --dump-outputs DIR also writes what the last timed end-to-end step returned.
 """
 import argparse
 import json
@@ -28,6 +28,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the tree may be read-only: nothing is written into it
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
@@ -70,6 +71,10 @@ def parse():
     ap.add_argument("--prepass", type=int, default=0, help="luma no-reference searches ahead of the chains (1) or inside them (0)")
     ap.add_argument("--level-chains", type=int, default=0, help="luma intra chains level-synchronously (1) instead of the dependency queue (0)")
     ap.add_argument("--shard", default="frames", choices=["frames", "sbrow"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the arrays the last timed end-to-end step returned (reconstruction, PVQ symbols, "
+                         "deringing levels) as DIR/<name>.npy, float32 or float64; arrays of more than %d values as "
+                         "the same seeded sample of that many values" % DUMP_LIMIT)
     return ap.parse_args()
 
 
@@ -402,6 +407,8 @@ def run_b200(args):
     e2e_loop(args.steps)
     ms_e2e = max_over_ranks((time.perf_counter() - t0) * 1e3)
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(slots[(args.steps - 1) % nslots].wait(), args.dump_outputs)
     clocks = sampler.stop() if rank == 0 else None
 
     # per-phase device times
@@ -515,6 +522,29 @@ def run_b200(args):
         dist.destroy_process_group()
     if out.get("parity_failed"):
         sys.exit(1)
+
+
+DUMP_LIMIT = 1 << 19
+
+
+def dump_outputs(out, dirname):
+    """Writes one step's result arrays (KeyframeEngine.wait()) as <name>.npy: integers of up to 16 bits as float32,
+    wider integers and doubles as float64, block descriptors as one float64 column per field.  An array of more than
+    DUMP_LIMIT values is sampled at DUMP_LIMIT positions drawn with a fixed seed from its size alone, so that two
+    builds given the same arguments write comparable samples.  `counts` holds the device queues' scheduling
+    counters, which vary from run to run, and is left out."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in sorted(out.items()):
+        if name == "counts":
+            continue
+        if a.dtype.names:
+            a = np.stack([a[f].astype(np.float64) for f in a.dtype.names], axis=-1)
+        flat = a.reshape(-1)
+        if flat.size > DUMP_LIMIT:
+            flat = flat[np.sort(np.random.default_rng(flat.size).integers(0, flat.size, DUMP_LIMIT))]
+        small = flat.dtype.kind in "iub" and flat.dtype.itemsize <= 2
+        np.save(os.path.join(dirname, name + ".npy"), flat.astype(np.float32 if small else np.float64))
 
 
 def load_profile_notes():

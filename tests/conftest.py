@@ -19,11 +19,11 @@ def port():
     return oracle_lib.load_port()
 
 
-@pytest.fixture(scope="session")
-def ref():
-    """The real reference, compiled by oracle/Makefile into oracle/_ref/ (may be absent)."""
-    from tests import oracle_lib
-    lib = oracle_lib.load_ref()
-    if lib is None:
-        pytest.skip("oracle/_ref/libdaala_ref.so not built (needs /root/reference)")
-    return lib
+@pytest.fixture
+def reference(request):
+    """What the reference build computes for the values this test compares: the library in oracle/_ref when it is
+    built, else the recorded CRC-32s of tests/golden/reference_pins.npz (tests/golden/pins.py)."""
+    from tests.golden import pins
+    r = pins.Reference(request.node.module.__name__ + "::" + request.node.name)
+    yield r
+    r.finish()

@@ -11,7 +11,11 @@ OD_QM_STRIDE = ((1 << 10) - 1) * 16 // 3              # OD_QM_OFFSET(OD_NBSIZES)
 
 
 def reference_qm(ref, hvs=True):
-    """state->qm / qm_inv exactly as od_init_qm (src/pvq.c:322) fills them."""
+    """state->qm / qm_inv exactly as od_init_qm (src/pvq.c:322) fills them; without the reference build, the same
+    tables as exported from it (daala_b200/data/qm_*.npy, checked against od_init_qm in tests/test_host_logic.py)."""
+    if ref is None:
+        from daala_b200 import pvq
+        return pvq.default_qm(hvs)
     qm = np.zeros(2 * OD_QM_STRIDE, np.int16)
     qm_inv = np.zeros(2 * OD_QM_STRIDE, np.int16)
     tbl = (ctypes.c_int * 64).in_dll(ref, "OD_QM8_Q4_HVS" if hvs else "OD_QM8_Q4_FLAT")

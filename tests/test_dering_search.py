@@ -13,7 +13,6 @@ import ctypes
 import numpy as np
 import pytest
 
-from tests import oracle_lib
 from tests.oracle_lib import addr
 
 LEVELS = 6
@@ -65,10 +64,7 @@ def coded_flags(bskip, nhsb, nvsb):
 
 
 @pytest.mark.parametrize("keyframe", [1, 0])
-def test_decision_matches_reference_cdf_model(keyframe):
-    ref = oracle_lib.load_ref()
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
+def test_decision_matches_reference_cdf_model(keyframe, reference):
     L = lib_decide()
     rng = np.random.default_rng(5 + keyframe)
     nhsb, nvsb = 7, 5
@@ -88,16 +84,22 @@ def test_decision_matches_reference_cdf_model(keyframe):
             bskip[16:32, 32:64] = 1            # two superblocks with every block skipped: not searched, not coded
             bskip = np.ascontiguousarray(bskip)
         lam = DERING_LAMBDA_SCALE * q * q
-        before = cdf_ref[:, -1].copy()
-        lv_ref, dist = ref_search(ref, src, ctmp, nhsb, nvsb, q, frame & 1, keyframe, lam, bskip, cdf_ref)
-        halved |= bool((cdf_ref[:, -1] < before).any())
+        before = cdf_ours[:, -1].copy()
+        search = {}
+
+        def ref_dist(ref):
+            # the reference's search runs frame after frame on its own CDFs (cdf_ref)
+            search["lv"], dist = ref_search(ref, src, ctmp, nhsb, nvsb, q, frame & 1, keyframe, lam, bskip, cdf_ref)
+            return dist
+        dist = np.ascontiguousarray(reference.value("dist%d" % frame, ref_dist))
         lv = np.zeros(nhsb * nvsb, np.uint8)
         coded = coded_flags(bskip, nhsb, nvsb) if bskip is not None else None
         r = L.daala_b200_dering_decide(addr(dist), nhsb, nvsb, keyframe, lam, addr(coded) if coded is not None else None,
                                        addr(cdf_ours), 128, addr(lv))
         assert r == 0
-        assert np.array_equal(lv, lv_ref), (frame, lv.reshape(nvsb, nhsb), lv_ref.reshape(nvsb, nhsb))
-        assert np.array_equal(cdf_ours, cdf_ref), frame
+        reference.check(lv, search.get("lv"), frame)
+        reference.check(cdf_ours, cdf_ref, frame)
+        halved |= bool((cdf_ours[:, -1] < before).any())
         if bskip is not None:
             assert lv.reshape(nvsb, nhsb)[1, 2] == 0 and lv.reshape(nvsb, nhsb)[1, 3] == 0
         seen |= set(lv.tolist())
@@ -109,11 +111,8 @@ def test_decision_matches_reference_cdf_model(keyframe):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("masking,keyframe,skips", [(0, 1, False), (1, 1, False), (1, 0, True)])
-def test_search_on_device_matches_reference(masking, keyframe, skips):
+def test_search_on_device_matches_reference(masking, keyframe, skips, reference):
     import torch
-    ref = oracle_lib.load_ref()
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
     L = lib_decide()
 
     class P(ctypes.Structure):
@@ -140,7 +139,12 @@ def test_search_on_device_matches_reference(masking, keyframe, skips):
             bskip[32:48, 16:48] = 1
             bskip = np.ascontiguousarray(bskip)
         lam = DERING_LAMBDA_SCALE * q * q
-        lv_ref, dist_ref = ref_search(ref, src, ctmp, nhsb, nvsb, q, masking, keyframe, lam, bskip, cdf_ref)
+        search = {}
+
+        def ref_dist(ref):
+            search["lv"], dist = ref_search(ref, src, ctmp, nhsb, nvsb, q, masking, keyframe, lam, bskip, cdf_ref)
+            return dist
+        dist_ref = reference.value("dist%d" % frame, ref_dist)
         d_etmp = torch.from_numpy(ctmp.astype(np.int16)).cuda()
         d_src = torch.from_numpy(src).cuda()
         d_skip = torch.from_numpy(bskip).cuda() if bskip is not None else None
@@ -152,7 +156,7 @@ def test_search_on_device_matches_reference(masking, keyframe, skips):
         assert L.daala_b200_dering_search(ctypes.byref(prm), addr(cdf_ours), 128, addr(lv), addr(dist), s) == 0
         coded = coded_flags(bskip, nhsb, nvsb).astype(bool) if bskip is not None else np.ones(nsb, bool)
         np.testing.assert_allclose(dist[:, coded], dist_ref[:, coded], rtol=1e-12, atol=0)
-        assert np.array_equal(lv, lv_ref), (frame, np.flatnonzero(lv != lv_ref))
-        assert np.array_equal(cdf_ours, cdf_ref)
+        reference.check(lv, search.get("lv"), frame)
+        reference.check(cdf_ours, cdf_ref, frame)
         seen |= set(lv.tolist())
     assert len(seen) >= 3, seen

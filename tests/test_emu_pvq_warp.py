@@ -1,7 +1,7 @@
 """The warp-per-band PVQ quantiser of the device (daala_b200/csrc/pvq_warp.cuh) compiled for the host
 on a SIMT emulation (tests/emu/simt_emu.h: 32 fibres, warp collectives as rendezvous) and pinned
-against the reference build's pvq_theta -- the same source the CUDA kernels include, so the candidate
-parallelisation, the event order and the redux-screened pulse search are checked on the CPU."""
+against the reference build's pvq_theta (or the outputs recorded from it) -- the same source the CUDA
+kernels include, so the candidate parallelisation, the event order and the redux-screened pulse search are checked on the CPU."""
 import ctypes
 import os
 import subprocess
@@ -9,7 +9,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from tests import oracle_lib, pvq_cases
+from tests import pvq_cases
 from tests.oracle_lib import addr
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -48,11 +48,6 @@ def _run(emu, c, qm, qm_inv):
     return dict(gain=g, itheta=it.value, max_theta=mt.value, k=vk.value, y=y[:ny].copy(), out=out, skip_diff=sd.value)
 
 
-def _same(a, b):
-    return (all(a[k] == b[k] for k in ("gain", "itheta", "max_theta", "k", "skip_diff")) and np.array_equal(a["y"], b["y"])
-            and np.array_equal(a["out"], b["out"]))
-
-
 # the second build lowers the "products are exact" bound so that the literal-scan path of the plain
 # pulses (taken on the device only when a product could exceed 2^53) runs on ordinary inputs
 # fourth run: keyframe luma with the no-reference half searched ahead of time (the engine's prepass);
@@ -62,8 +57,7 @@ def _same(a, b):
                                                     ("libpvq_warp_emu_scan.so", ["-DDAALA_B200_PVQ_EXACT_BOUND=1e12"], (1,), False),
                                                     ("libpvq_warp_emu.so", [], (4,), True),
                                                     ("libpvq_warp_emu.so", [], (5,), "prepass")])
-def test_warp_quantiser_matches_reference(name, extra, seeds, split, monkeypatch):
-    ref = oracle_lib.load_ref()
+def test_warp_quantiser_matches_reference(name, extra, seeds, split, monkeypatch, reference):
     emu = _build(name, extra)
     # "prepass": keyframe luma bands with their no-reference events searched ahead of time and imported
     monkeypatch.delenv("DAALA_B200_EMU_SPLIT", raising=False)
@@ -72,14 +66,14 @@ def test_warp_quantiser_matches_reference(name, extra, seeds, split, monkeypatch
         monkeypatch.setenv("DAALA_B200_EMU_PREPASS", "1")
     elif split:
         monkeypatch.setenv("DAALA_B200_EMU_SPLIT", "1")
-    qm, qm_inv = pvq_cases.reference_qm(ref)
+    qm, qm_inv = pvq_cases.reference_qm(reference.lib)
     stats = (ctypes.c_longlong * 4).in_dll(emu, "daala_b200_pvq_warp_stats")
     n = 0
     for seed in seeds:
         for c in pvq_cases.cases(seed=seed, per_combo=3):
-            want = pvq_cases.run_theta(ref, "ref", c, qm, qm_inv)
             got = _run(emu, c, qm, qm_inv)
-            assert _same(want, got), ({k: c[k] for k in ("n", "kind", "is_keyframe", "pli", "beta", "q0", "lam")}, want, got)
+            reference.check(got, lambda ref: pvq_cases.run_theta(ref, "ref", c, qm, qm_inv),
+                            {k: c[k] for k in ("n", "kind", "is_keyframe", "pli", "beta", "q0", "lam")})
             n += 1
     # coverage: unique-contender fast path, both exact fallbacks, and (second build) the literal scan
     assert n >= 400 and stats[0] > 0 and stats[1] > 0 and stats[2] > 0
@@ -87,11 +81,10 @@ def test_warp_quantiser_matches_reference(name, extra, seeds, split, monkeypatch
         assert stats[3] > 0
 
 
-def test_warp_quantiser_large_k():
+def test_warp_quantiser_large_k(reference):
     """Fine quantisers on large vectors: K in the hundreds to thousands (all-RDO searches, 64-bit sums)."""
-    ref = oracle_lib.load_ref()
     emu = _build("libpvq_warp_emu.so", [])
-    qm, qm_inv = pvq_cases.reference_qm(ref)
+    qm, qm_inv = pvq_cases.reference_qm(reference.lib)
     rng = np.random.default_rng(7)
     kmax = 0
     for q0 in (16, 40, 500, 620):
@@ -99,8 +92,7 @@ def test_warp_quantiser_large_k():
             for kf, pli in ((1, 0), (1, 1), (0, 0)):
                 x0, r0 = pvq_cases.make_band(rng, n, "big")
                 c = dict(n=n, kind="big", is_keyframe=kf, pli=pli, beta=4096, q0=q0, x0=x0, r0=r0, qm_off=5, lam=0.147)
-                want = pvq_cases.run_theta(ref, "ref", c, qm, qm_inv)
                 got = _run(emu, c, qm, qm_inv)
-                assert _same(want, got), (q0, n, kf, pli, want, got)
-                kmax = max(kmax, want["k"])
+                reference.check(got, lambda ref: pvq_cases.run_theta(ref, "ref", c, qm, qm_inv), (q0, n, kf, pli))
+                kmax = max(kmax, got["k"])
     assert kmax > 1000

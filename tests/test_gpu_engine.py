@@ -261,7 +261,7 @@ def test_engine_baseline_sizes_q72_match_oracle(size, maps):
     eng.close()
 
 
-def test_engine_dering_stage_matches_oracle():
+def test_engine_dering_stage_matches_oracle(reference):
     """daala_b200_kf_config.dering: the reconstruction through od_dering with caller-supplied per-superblock
     levels (the final application of src/encode.c:2812-2842 on keyframes: no block is marked skipped, luma
     directions re-used by chroma, chroma thresholds * 0.6, level 0 = untouched).  Oracle: the reference chain
@@ -269,9 +269,6 @@ def test_engine_dering_stage_matches_oracle():
     import ctypes
     from daala_b200 import engine
     from daala_b200.frame import Geometry
-    lib, prefix = _oracle()
-    if prefix != "ref":
-        pytest.skip("needs the reference build (od_apply_postfilter_frame_sbs)")
     port = oracle_lib.load_port()
     geom = Geometry(328, 200)
     q0, q4 = 72, np.full((3, 30), 16, np.uint8)
@@ -287,12 +284,15 @@ def test_engine_dering_stage_matches_oracle():
     base = float(q0) ** 0.84182
     Dir = (ctypes.c_int * 8) * 8
     a = oracle_lib.addr
-    for f in range(F):
+
+    def oracle(lib, f):
+        """Per plane the reconstruction through the frame driver's od_dering, then per plane the same through the
+        reference's SB-edge postfilter and the pinned deringing port."""
+        prefix = "ref"
         want = frame_oracle.keyframe_chain(lib, prefix, frames[f][0], geom, frames[f][1], q0, q4, 1)
         # the same through the oracle's frame driver (the reference's own od_dering), which bench.py uses
         want_d = frame_oracle.keyframe_chain(lib, prefix, frames[f][0], geom, frames[f][1], q0, q4, 1, dering_levels=levels[f])
-        for pli in range(3):
-            assert np.array_equal(out["recon%d" % pli][f], want_d[pli]["recon"]), ("dering recon vs od_dering", f, pli)
+        recs = [want_d[pli]["recon"] for pli in range(3)]
         dirs = {}
         for pli in range(3):
             xdec = 1 if pli else 0
@@ -317,14 +317,19 @@ def test_engine_dering_stage_matches_oracle():
                     port.port_dering(a(yb), sb, a(x16, sby * sb * w + sbx * sb), w, 8, 8, sbx, sby, geom.nhsb, geom.nvsb,
                                      xdec, d, pli, a(bskip, (sby * units) * skip_stride + sbx * units), skip_stride, thr, 1, 4)
                     y16[sby * sb:(sby + 1) * sb, sbx * sb:(sbx + 1) * sb] = yb
-            rec = np.clip(((y16.astype(np.int32) + 8) >> 4) + 128, 0, 255).astype(np.uint8)
-            got = out["recon%d" % pli][f]
-            assert np.array_equal(got, rec), ("dering recon", f, pli, int((got != rec).sum()))
+            recs.append(np.clip(((y16.astype(np.int32) + 8) >> 4) + 128, 0, 255).astype(np.uint8))
+        return recs
+    for f in range(F):
+        want = oracle(reference.lib, f) if reference.lib is not None else [None] * 6
+        for pli in range(3):
+            reference.check(out["recon%d" % pli][f], want[pli], ("dering recon vs od_dering", f, pli))
+        for pli in range(3):
+            reference.check(out["recon%d" % pli][f], want[3 + pli], ("dering recon", f, pli))
     eng.close()
 
 
 @pytest.mark.parametrize("q0", [72, 38])
-def test_engine_dering_search_matches_reference(q0):
+def test_engine_dering_search_matches_reference(q0, reference):
     """daala_b200_kf_config.dering = 2: the engine searches the deringing levels itself (src/encode.c:2708-2811: five
     filtered candidates and the unfiltered reconstruction scored by od_compute_dist + lambda * adaptive-CDF rate, one
     decision thread per frame) and applies them.  Oracle: the reference chain up to the SB-edge postfilter (ctmp),
@@ -334,9 +339,6 @@ def test_engine_dering_search_matches_reference(q0):
     from daala_b200 import engine
     from daala_b200.frame import Geometry
     from tests import test_dering_search as ds
-    lib, prefix = _oracle()
-    if prefix != "ref":
-        pytest.skip("needs the reference build (od_compute_dist, od_dering, od_encode_cdf_*)")
     geom = Geometry(328, 200)
     q4 = np.full((3, 30), 16, np.uint8)
     F = 3
@@ -346,7 +348,9 @@ def test_engine_dering_search_matches_reference(q0):
     got_levels = out["dering_levels"].copy()
     a = oracle_lib.addr
     seen = set()
-    for f in range(F):
+
+    def levels(lib, f):
+        prefix = "ref"
         want = frame_oracle.keyframe_chain(lib, prefix, frames[f][0], geom, frames[f][1], q0, q4, 1)
         c = frame_oracle.inverse_plane(lib, prefix, want[0]["dq"], geom, 0, frames[f][1], 1, lapped_only=True)
         c = np.ascontiguousarray(c, np.int32)
@@ -355,11 +359,18 @@ def test_engine_dering_search_matches_reference(q0):
         cdf[:] = 32 * np.arange(1, 7, dtype=np.uint16)
         src = np.ascontiguousarray(frames[f][0][0], np.uint8)
         lv_ref, _ = ds.ref_search(lib, src, c, geom.nhsb, geom.nvsb, q0, 1, 1, eng.dering_lambda, None, cdf)
-        lv_ref = lv_ref.reshape(geom.nvsb, geom.nhsb)
-        assert np.array_equal(got_levels[f], lv_ref), (f, got_levels[f], lv_ref)
-        seen |= set(lv_ref.ravel().tolist())
-        want_d = frame_oracle.keyframe_chain(lib, prefix, frames[f][0], geom, frames[f][1], q0, q4, 1, dering_levels=lv_ref)
+        return lv_ref.reshape(geom.nvsb, geom.nhsb)
+
+    def recons(lib, f):
+        want_d = frame_oracle.keyframe_chain(lib, "ref", frames[f][0], geom, frames[f][1], q0, q4, 1,
+                                             dering_levels=got_levels[f])
+        return [want_d[pli]["recon"] for pli in range(3)]
+    for f in range(F):
+        reference.check(got_levels[f], lambda lib: levels(lib, f), f)
+        seen |= set(got_levels[f].ravel().tolist())
+        want = recons(reference.lib, f) if reference.lib is not None else [None] * 3
         for pli in range(3):
-            assert np.array_equal(out["recon%d" % pli][f], want_d[pli]["recon"]), ("recon at the searched levels", f, pli)
+            # the reconstruction at the levels the reference chose (equal to the engine's, as checked)
+            reference.check(out["recon%d" % pli][f], want[pli], ("recon at the searched levels", f, pli))
     assert len(seen) >= 2, seen
     eng.close()

@@ -194,14 +194,24 @@ def _random_mv_grid(rng, nv, nh, max_mv=200):
     return valid, mv
 
 
-def test_frame_obmc_prediction_matches_reference_state_mc_predict():
+def _state_mc_predict(ref, W, H, ref_y, ref_u, ref_v, valid, mv):
+    """The three planes od_state_mc_predict predicts on a real od_state (oracle/ref_hooks_mc.c); None per plane
+    without the reference build."""
+    if ref is None:
+        return [None] * 3
+    outs = [np.zeros((H, W), np.uint8), np.zeros((H // 2, W // 2), np.uint8), np.zeros((H // 2, W // 2), np.uint8)]
+    rc = ref.oracle_ref_state_mc_predict(W, H, addr(ref_y), addr(ref_u), addr(ref_v),
+                                         addr(np.ascontiguousarray(valid.astype(np.uint8))),
+                                         addr(np.ascontiguousarray(mv)), addr(outs[0]), addr(outs[1]), addr(outs[2]))
+    assert rc == 0
+    return outs
+
+
+def test_frame_obmc_prediction_matches_reference_state_mc_predict(reference):
     """MV grid -> block list (daala_b200/mvgrid.py) -> k_obmc_blocks for all three planes against
     the reference's od_state_mc_predict driven on a real od_state (oracle/ref_hooks_mc.c)."""
     import torch
     from daala_b200 import mc, mvgrid
-    lib, prefix = _oracle()
-    if prefix != "ref":
-        pytest.skip("needs the reference build (od_state_mc_predict)")
     rng = np.random.default_rng(21)
     W, H = 256, 192
     cur, ref_y = _frames(seed=6, h=H, w=W)
@@ -209,11 +219,7 @@ def test_frame_obmc_prediction_matches_reference_state_mc_predict():
     ref_v = np.ascontiguousarray(ref_y[1::2, 1::2])
     nv, nh = H // 8, W // 8
     valid, mv = _random_mv_grid(rng, nv, nh)
-    outs = [np.zeros((H, W), np.uint8), np.zeros((H // 2, W // 2), np.uint8), np.zeros((H // 2, W // 2), np.uint8)]
-    rc = lib.oracle_ref_state_mc_predict(W, H, addr(ref_y), addr(ref_u), addr(ref_v),
-                                         addr(np.ascontiguousarray(valid.astype(np.uint8))),
-                                         addr(np.ascontiguousarray(mv)), addr(outs[0]), addr(outs[1]), addr(outs[2]))
-    assert rc == 0
+    outs = _state_mc_predict(reference.lib, W, H, ref_y, ref_u, ref_v, valid, mv)
     for pli, refp in enumerate((ref_y, ref_u, ref_v)):
         xdec = 1 if pli else 0
         blocks = mvgrid.block_list(valid, mv, xdec=xdec)
@@ -221,10 +227,10 @@ def test_frame_obmc_prediction_matches_reference_state_mc_predict():
         dst = torch.zeros(refp.shape, dtype=torch.uint8, device="cuda:0")
         mc.predict_blocks(rp, dst, mc.to_device(blocks), len(blocks))
         got = dst.cpu().numpy()
-        assert np.array_equal(got, outs[pli]), "plane %d: %d mismatches" % (pli, int((got != outs[pli]).sum()))
+        reference.check(got, outs[pli], "plane %d" % pli)
 
 
-def test_inter_frame_chain_mv_grid_to_pvq_matches_reference():
+def test_inter_frame_chain_mv_grid_to_pvq_matches_reference(reference):
     """The inter-frame hot path end to end on the device: MV grid -> OBMC prediction of all planes
     (k_obmc_blocks) -> forward transform of the prediction (the reference's mdtmp planes,
     src/encode.c:2566-2573) -> forward transform of the source -> PVQ against that prediction ->
@@ -236,8 +242,6 @@ def test_inter_frame_chain_mv_grid_to_pvq_matches_reference():
     from daala_b200.pipeline import HotPath
     from tests import frame_oracle
     lib, prefix = _oracle()
-    if prefix != "ref":
-        pytest.skip("needs the reference build (od_state_mc_predict)")
     rng = np.random.default_rng(33)
     W, H = 256, 192
     geom = Geometry(W, H)
@@ -247,12 +251,7 @@ def test_inter_frame_chain_mv_grid_to_pvq_matches_reference():
     cur = [cur_y, np.ascontiguousarray(cur_y[::2, ::2][:, ::-1]), np.ascontiguousarray(cur_y[1::2, 1::2])]
     valid, mv = _random_mv_grid(rng, H // 8, W // 8)
     # reference prediction
-    pred_ref = [np.zeros((H, W), np.uint8), np.zeros((H // 2, W // 2), np.uint8), np.zeros((H // 2, W // 2), np.uint8)]
-    rc = lib.oracle_ref_state_mc_predict(W, H, addr(ref_y), addr(ref_u), addr(ref_v),
-                                         addr(np.ascontiguousarray(valid.astype(np.uint8))),
-                                         addr(np.ascontiguousarray(mv)), addr(pred_ref[0]), addr(pred_ref[1]),
-                                         addr(pred_ref[2]))
-    assert rc == 0
+    pred_ref = _state_mc_predict(reference.lib, W, H, ref_y, ref_u, ref_v, valid, mv)
     # device chain
     bsize = synth.block_size_map(geom, "mixed", seed=12)
     q4 = np.full((3, 30), 20, np.uint8)
@@ -274,9 +273,11 @@ def test_inter_frame_chain_mv_grid_to_pvq_matches_reference():
     qm, qm_inv = pvq.default_qm(True)
     coded = 0
     for pli in range(3):
-        assert np.array_equal(pred.pixels[pli][0].cpu().numpy(), pred_ref[pli]), "prediction plane %d" % pli
+        pred_dev = pred.pixels[pli][0].cpu().numpy()
+        reference.check(pred_dev, pred_ref[pli], "prediction plane %d" % pli)
         d = frame_oracle.forward_plane(lib, prefix, cur[pli], geom, pli, bsize, 0)
-        md = frame_oracle.forward_plane(lib, prefix, pred_ref[pli], geom, pli, bsize, 0)
+        # the device's prediction, equal to the reference's as checked
+        md = frame_oracle.forward_plane(lib, prefix, pred_dev, geom, pli, bsize, 0)
         dq, stats = frame_oracle.pvq_plane(lib, prefix, d, md, geom, pli, bsize, 45, 0, 1, 0.147, qm, qm_inv, q4)
         coded += int(stats[0])
         assert np.array_equal(hp.fb.coeffs[pli][0].cpu().numpy(), dq), "quantised plane %d" % pli
@@ -285,7 +286,7 @@ def test_inter_frame_chain_mv_grid_to_pvq_matches_reference():
     assert coded > 0
 
 
-def test_bma_candidate_cost_matches_reference():
+def test_bma_candidate_cost_matches_reference(reference):
     """daala_b200_mv_bma_sad against the reference's own od_mv_est_bma_sad (static, src/mcenc.c:2224) run on
     a real od_state: all three planes, chroma >> 2, blocks hanging over every picture edge (od_enc_sad's
     clipping, including the negative origins of centred BMA blocks), every block size, fractional and
@@ -295,9 +296,6 @@ def test_bma_candidate_cost_matches_reference():
     from daala_b200 import _native, synth
     from daala_b200.frame import Geometry
     L = _native.lib()
-    ref = oracle_lib.load_ref()
-    if ref is None:
-        pytest.skip("needs oracle/_ref")
     pic_w, pic_h = 200, 130
     geom = Geometry(pic_w, pic_h)
     cur, _ = synth.frame(pic_w, pic_h, f=3)
@@ -317,10 +315,12 @@ def test_bma_candidate_cost_matches_reference():
     jobs = np.array(jobs, np.int32)
     a = oracle_lib.addr
     for use_chroma in (1, 0):
-        want = np.zeros(len(jobs), np.int32)
-        rc = ref.oracle_ref_bma_sad(pic_w, pic_h, a(cur[0]), a(cur[1]), a(cur[2]), a(prev[0]), a(prev[1]), a(prev[2]),
-                                    use_chroma, a(jobs), len(jobs), a(want))
-        assert rc == 0
+        def bma_sad(ref):
+            want = np.zeros(len(jobs), np.int32)
+            rc = ref.oracle_ref_bma_sad(pic_w, pic_h, a(cur[0]), a(cur[1]), a(cur[2]), a(prev[0]), a(prev[1]), a(prev[2]),
+                                        use_chroma, a(jobs), len(jobs), a(want))
+            assert rc == 0
+            return want
         pad = 96
         dev_cur, dev_ref, cs, rs, cptr, rptr = [], [], [], [], [], []
         for p in range(3):
@@ -342,12 +342,10 @@ def test_bma_candidate_cost_matches_reference():
                                      d_jobs.data_ptr(), len(jobs), d_out.data_ptr(), None)
         assert rc == 0
         torch.cuda.synchronize()
-        got = d_out.cpu().numpy()
-        bad = np.nonzero(got != want)[0]
-        assert len(bad) == 0, (use_chroma, len(bad), jobs[bad[:5]].tolist(), got[bad[:5]].tolist(), want[bad[:5]].tolist())
+        reference.check(d_out.cpu().numpy(), bma_sad, use_chroma)
 
 
-def test_obmc_candidate_cost_matches_reference():
+def test_obmc_candidate_cost_matches_reference(reference):
     """daala_b200_mv_est_sad against the reference's own od_mv_est_sad (static, src/mcenc.c:2267) on a real
     od_state with a random MV grid: OBMC prediction of all three planes from the grid (every outside corner /
     split state the grid produces, all block sizes) + od_enc_sad with clipping at the picture edge, chroma >> 2."""
@@ -356,9 +354,6 @@ def test_obmc_candidate_cost_matches_reference():
     from daala_b200 import _native, mc, mvgrid, synth
     from daala_b200.frame import Geometry
     L = _native.lib()
-    ref = oracle_lib.load_ref()
-    if ref is None:
-        pytest.skip("needs oracle/_ref")
     pic_w, pic_h = 200, 130
     geom = Geometry(pic_w, pic_h)
     W, H = geom.frame_w, geom.frame_h
@@ -374,10 +369,12 @@ def test_obmc_candidate_cost_matches_reference():
     vmap = np.ascontiguousarray(valid.astype(np.uint8))
     mvc = np.ascontiguousarray(mv)
     for use_chroma in (1, 0):
-        want = np.zeros(len(jobs), np.int32)
-        rc = ref.oracle_ref_mv_est_sad(pic_w, pic_h, a(cur[0]), a(cur[1]), a(cur[2]), a(prev[0]), a(prev[1]), a(prev[2]),
-                                       a(vmap), a(mvc), use_chroma, a(jobs), len(jobs), a(want))
-        assert rc == 0
+        def mv_est_sad(ref):
+            want = np.zeros(len(jobs), np.int32)
+            rc = ref.oracle_ref_mv_est_sad(pic_w, pic_h, a(cur[0]), a(cur[1]), a(cur[2]), a(prev[0]), a(prev[1]),
+                                           a(prev[2]), a(vmap), a(mvc), use_chroma, a(jobs), len(jobs), a(want))
+            assert rc == 0
+            return want
         blocks = np.zeros((len(jobs), 3), mc.MC_BLOCK_DTYPE)
         for p in range(3):
             blocks[:, p] = mvgrid.blocks_for(vx, vy, l, oc, s, mv, xdec=1 if p else 0)
@@ -402,7 +399,5 @@ def test_obmc_candidate_cost_matches_reference():
                                      d_blocks.data_ptr(), len(jobs), d_out.data_ptr(), None)
         assert rc == 0
         torch.cuda.synchronize()
-        got = d_out.cpu().numpy()
-        bad = np.nonzero(got != want)[0]
-        assert len(bad) == 0, (use_chroma, len(bad), len(jobs), jobs[bad[:5]].tolist(), got[bad[:5]].tolist(), want[bad[:5]].tolist())
+        reference.check(d_out.cpu().numpy(), mv_est_sad, use_chroma)
     assert len(jobs) > 50 and len(np.unique(l)) >= 3
